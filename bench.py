@@ -529,6 +529,8 @@ def run_supir(args):
     step_ms = t0.elapsed_time(t1) / args.steps
     lc1 = _native.launch_count() + net.replayed_launches
     clk = clocks.stop() if rank == 0 else None
+    # the latent the last timed sampler step returned; the e2e steps below overwrite run.x
+    dumped = run.x.detach().float().cpu() if args.dump_outputs else None
     # ---- e2e steps: host latent in, host latent out, every step ----
     x_host = run.x.detach().cpu().pin_memory()
     res_host = torch.empty_like(x_host).pin_memory()
@@ -643,6 +645,9 @@ def run_supir(args):
     }
     if cpu is not None:
         line["cpu_baseline"] = cpu
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "latent.npy"), dumped.numpy())
     print(json.dumps(line))
     if world > 1:
         dist.barrier()
@@ -658,7 +663,11 @@ def main():
     ap.add_argument("--config", default="cfg3", choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-full-run", action="store_true", help="skip the one real batchify_sample run of the whole configuration")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the latent the last timed sampler step returned to DIR/latent.npy (float32; rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "supir_b200" else args.warmup
     if args.impl == "reference":
         run_reference(args)

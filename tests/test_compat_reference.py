@@ -1,80 +1,67 @@
-"""When the reference checkout is present (build container only): compat.install() makes the reference's own factory
-resolve the hot-path targets to this package's classes, and the live reference still agrees with the committed fixtures."""
+"""compat.install() against the reference's module layout, the reference's model configurations through this package's factory,
+and PreparedConditioner against the reference class. The reference is not part of this repository: its three configurations are
+stored unedited under tests/golden/options/, and the names its modules define and what its PreparedConditioner returns are
+recorded in tests/golden/reference_io.npz (tests/golden/make_reference_io.py)."""
+import importlib
+import json
 import os
 import sys
+import types
 
+import numpy as np
 import pytest
 
-sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
-import ref_stubs  # noqa: E402
+GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
+sys.path.insert(0, GOLDEN)
+REF =np.load(os.path.join(GOLDEN, "reference_io.npz"))
+REF_NAMES = json.loads(str(REF["compat_names"]))
 
-pytestmark = pytest.mark.skipif(not ref_stubs.reference_available(), reason="/root/reference not present (GPU box)")
 
-
-def test_install_rebinds_reference_targets():
-    ns = ref_stubs.import_reference()
-    import sgm.util as sgm_util
-    import supir_b200.compat as compat
-    saved = {}
-    import importlib
-    for modname, attrs in compat.PATCHES.items():
-        try:
-            mod = importlib.import_module(modname)
-        except Exception:
-            continue
+@pytest.fixture()
+def reference_modules(monkeypatch):
+    """Stand-ins for the reference modules compat.install() patches, each holding a placeholder under every name the reference's
+    module defines; they leave sys.modules when the test ends."""
+    placeholders = {}
+    for modname, attrs in REF_NAMES.items():
+        parts = modname.split(".")
+        for i in range(1, len(parts) + 1):
+            name = ".".join(parts[:i])
+            if name not in placeholders:
+                monkeypatch.setitem(sys.modules, name, types.ModuleType(name))
+                placeholders[name] = {}
+        mod = sys.modules[modname]
         for a in attrs:
-            saved[(modname, a)] = getattr(mod, a, None)
-    try:
-        done = compat.install(strict=False)
-        assert ("sgm.modules.diffusionmodules.sampling", "TiledRestoreEDMSampler") in done
-        assert ("SUPIR.modules.SUPIR_v0", "LightGLVUNet") in done
-        smp = sgm_util.instantiate_from_config({
-            "target": "sgm.modules.diffusionmodules.sampling.TiledRestoreEDMSampler",
-            "params": {"num_steps": 5, "restore_cfg": 4.0, "s_churn": 0, "s_noise": 1.003, "tile_size": 128, "tile_stride": 64, "device": "cpu",
-                       "discretization_config": {"target": "sgm.modules.diffusionmodules.discretizer.LegacyDDPMDiscretization"},
-                       "guider_config": {"target": "sgm.modules.diffusionmodules.guiders.LinearCFG", "params": {"scale": 7.5, "scale_min": 4.0}}}})
-        assert type(smp).__module__ == "supir_b200.sampling" and type(smp.guider).__module__ == "supir_b200.guiders"
-        cls = sgm_util.get_obj_from_str("SUPIR.modules.SUPIR_v0.GLVControl")
-        assert cls.__module__ == "supir_b200.nets"
-        assert sgm_util.get_obj_from_str("sgm.modules.diffusionmodules.wrappers.ControlWrapper").__module__ == "supir_b200.wrappers"
-    finally:
-        for (modname, a), v in saved.items():
-            if v is not None:
-                setattr(importlib.import_module(modname), a, v)
+            placeholders[modname][a] = type(a, (), {"__module__": modname})
+            setattr(mod, a, placeholders[modname][a])
+    return placeholders
 
 
-def test_install_conditioner_is_opt_in_and_resolves_through_the_reference_factory():
-    ref_stubs.import_reference()
-    import importlib
-    import sgm.util as sgm_util
+def test_install_rebinds_reference_targets(reference_modules):
+    import supir_b200.compat as compat
+    for modname, attrs in dict(compat.PATCHES, **compat.CONDITIONER_PATCHES).items():
+        assert set(attrs) <= set(REF_NAMES[modname]), f"compat patches names {modname} does not define"
+    done = compat.install(strict=False)
+    assert sorted(done) == sorted((m, a) for m, attrs in compat.PATCHES.items() for a in attrs)
+    for m, a in done:
+        assert getattr(importlib.import_module(m), a) is compat._resolve(compat.PATCHES[m][a])
+    # what the reference's get_obj_from_str / instantiate_from_config do with a target string: import the module, getattr
+    smp_cls = getattr(importlib.import_module("sgm.modules.diffusionmodules.sampling"), "TiledRestoreEDMSampler")
+    smp = smp_cls(num_steps=5, restore_cfg=4.0, s_churn=0, s_noise=1.003, tile_size=128, tile_stride=64, device="cpu",
+                  discretization_config={"target": "sgm.modules.diffusionmodules.discretizer.LegacyDDPMDiscretization"},
+                  guider_config={"target": "sgm.modules.diffusionmodules.guiders.LinearCFG", "params": {"scale": 7.5, "scale_min": 4.0}})
+    assert type(smp).__module__ == "supir_b200.sampling" and type(smp.guider).__module__ == "supir_b200.guiders"
+    assert getattr(importlib.import_module("SUPIR.modules.SUPIR_v0"), "GLVControl").__module__ == "supir_b200.nets"
+    assert getattr(importlib.import_module("sgm.modules.diffusionmodules.wrappers"), "ControlWrapper").__module__ == "supir_b200.wrappers"
+
+
+def test_install_conditioner_is_opt_in_and_resolves_through_the_reference_factory(reference_modules):
     import supir_b200.compat as compat
     E = importlib.import_module("sgm.modules.encoders.modules")
-    saved = {}
-    for modname, attrs in dict(compat.PATCHES, **compat.CONDITIONER_PATCHES).items():      # install() rebinds all of these
-        try:
-            m = importlib.import_module(modname)
-        except Exception:
-            continue
-        saved.update({(m, a): getattr(m, a) for a in attrs if hasattr(m, a)})
-    try:
-        compat.install(strict=False)
-        assert E.FrozenCLIPEmbedder.__module__ == "sgm.modules.encoders.modules"          # untouched by default
-        compat.install(strict=False, conditioner=True)
-        cls = sgm_util.get_obj_from_str("sgm.modules.GeneralConditionerWithControl")
-        assert cls.__module__ == "supir_b200.conditioner"
-        assert sgm_util.get_obj_from_str("sgm.modules.encoders.modules.FrozenOpenCLIPEmbedder2").__module__ == "supir_b200.conditioner"
-    finally:
-        for (m, a), v in saved.items():
-            setattr(m, a, v)
-
-
-def test_reference_still_matches_bookkeeping_fixture():
-    import json
-    ns = ref_stubs.import_reference()
-    with open(os.path.join(os.path.dirname(__file__), "golden", "bookkeeping.json")) as f:
-        book = json.load(f)
-    for case in book["sliding_windows"]:
-        assert [list(c) for c in ns.sampling._sliding_windows(*case["args"])] == case["windows"]
+    compat.install(strict=False)
+    assert E.FrozenCLIPEmbedder is reference_modules["sgm.modules.encoders.modules"]["FrozenCLIPEmbedder"]   # untouched by default
+    compat.install(strict=False, conditioner=True)
+    assert getattr(importlib.import_module("sgm.modules"), "GeneralConditionerWithControl").__module__ == "supir_b200.conditioner"
+    assert getattr(E, "FrozenOpenCLIPEmbedder2").__module__ == "supir_b200.conditioner"
 
 
 def test_every_reference_yaml_instantiates_through_this_packages_factory():
@@ -84,7 +71,7 @@ def test_every_reference_yaml_instantiates_through_this_packages_factory():
     import glob
     import torch
     from supir_b200.config import instantiate_from_config, load_yaml
-    paths = sorted(glob.glob(os.path.join(ref_stubs.REFERENCE_ROOT, "options", "*.yaml")))
+    paths = sorted(glob.glob(os.path.join(GOLDEN, "options", "*.yaml")))
     assert len(paths) >= 3
     samplers = set()
     for path in paths:
@@ -106,21 +93,17 @@ def test_every_reference_yaml_instantiates_through_this_packages_factory():
 def test_prepared_conditioner_matches_the_reference_class(tmp_path):
     """sgm.modules.PreparedConditioner (modules.py:246-290): conditions loaded from .pth files and repeated to the batch."""
     import torch
-    ref_stubs.import_reference()
-    import importlib
-    E = importlib.import_module("sgm.modules.encoders.modules")
+    import reference_cases
     from supir_b200.config import instantiate_from_config
-    g = torch.Generator().manual_seed(0)
-    c = {"crossattn": torch.randn(1, 77, 32, generator=g), "vector": torch.randn(1, 16, generator=g)}
-    uc = {"crossattn": torch.randn(1, 77, 32, generator=g), "vector": torch.randn(1, 16, generator=g)}
+    c, uc, batch = reference_cases.prepared_conditioner_inputs()
     torch.save(c, tmp_path / "c.pth")
     torch.save(uc, tmp_path / "uc.pth")
-    batch = {"control": torch.randn(3, 4, 8, 8, generator=g)}
-    for un in (str(tmp_path / "uc.pth"), None):
+    for tag, un in (("uc", str(tmp_path / "uc.pth")), ("none", None)):
         mine = instantiate_from_config({"target": "sgm.modules.PreparedConditioner", "params": {"cond_pth": str(tmp_path / "c.pth"), "un_cond_pth": un}})
-        ref = E.PreparedConditioner(str(tmp_path / "c.pth"), un)
-        assert type(mine).__module__ == "supir_b200.conditioner" and type(ref).__module__ == "sgm.modules.encoders.modules"
-        (a, au), (b, bu) = mine.get_unconditional_conditioning(batch), ref.get_unconditional_conditioning(batch)
-        assert a.keys() == b.keys() and all(torch.equal(a[k], b[k]) for k in a)
-        assert (au is None and bu is None) or (au.keys() == bu.keys() and all(torch.equal(au[k], bu[k]) for k in au))
-        assert mine.state_dict().keys() == ref.state_dict().keys()
+        assert type(mine).__module__ == "supir_b200.conditioner"
+        a, au = mine.get_unconditional_conditioning(batch)
+        want = {k[len(f"prepared_{tag}_c_"):]: REF[k] for k in REF.files if k.startswith(f"prepared_{tag}_c_")}
+        want_u = {k[len(f"prepared_{tag}_uc_"):]: REF[k] for k in REF.files if k.startswith(f"prepared_{tag}_uc_")}
+        assert sorted(a) == sorted(want) and all(np.array_equal(a[k].numpy(), want[k]) for k in a)
+        assert (au is None and not want_u) or (sorted(au) == sorted(want_u) and all(np.array_equal(au[k].numpy(), want_u[k]) for k in au))
+        assert sorted(mine.state_dict().keys()) == json.loads(str(REF[f"prepared_{tag}_keys"]))

@@ -1,26 +1,29 @@
-"""The drop-in claim, end to end, in the build container: the REFERENCE's own engine class (SUPIR/models/SUPIR_model.py
-`SUPIRModel(DiffusionEngine)`, imported unmodified from /root/reference) is built twice from the same YAML-shaped config and the
-same weights — once as is (pure PyTorch reference), once after `supir_b200.compat.install(conditioner=True)` so that every
-`target:` string resolves to this package's classes — and `batchify_sample(image, prompts, ...)` is run on both: stage-1
-encode / decode, re-encode, text conditioning from prompt strings, the EDM restore sampler driving the reference's opaque denoiser
-lambda (SUPIR_model.py:123-125), final decode, also with the tiled VAE hooks (`init_tile_vae`), the tiled sampler and per-window prompts.
+"""The drop-in claim, end to end, on CPU: this package's engine (supir_b200.model.SUPIRModel) is built from a YAML-shaped config
+and the same weights as the reference's own engine class (SUPIR/models/SUPIR_model.py `SUPIRModel(DiffusionEngine)`), and
+`batchify_sample(image, prompts, ...)` is run: stage-1 encode / decode, re-encode, text conditioning from prompt strings, the EDM
+restore sampler, final decode, also with the tiled VAE hooks (`init_tile_vae`), the tiled sampler and per-window prompts, then the
+stage-1-only denoise. The reference engine's outputs on the same config, weights, inputs and noise sequence (a fixed seeded sample
+of each, with its shape) are stored in
+tests/golden/dropin_engine.npz (tests/golden/make_reference_io.py), together with its state_dict layout and sigma table.
 No GPU here, so the backend's kernels are the plain-torch stand-ins of tests/cpu_ops.py (bf16 storage where the kernels store
-bf16): what this pins is that the reference's orchestration code runs UNCHANGED on the backend's classes — constructor
-signatures, attributes it pokes (`model.dtype`, `load_control_model`, re-bindable `.forward` / `.original_forward`,
-`sampler_config.params.*`), call signatures, RNG order — and produces the reference's result within the bf16 tolerance."""
+bf16): what this pins is the engine's state_dict layout, its call signatures and RNG order, and that it produces the reference's
+result within the bf16 tolerance."""
 import copy
+import json
 import os
 import sys
 
+import numpy as np
 import pytest
 import torch
 
 sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
-import ref_stubs  # noqa: E402
+import reference_cases  # noqa: E402
 from weights import cond_tokens, make_state_dict, randn  # noqa: E402
 
-pytestmark = pytest.mark.skipif(not ref_stubs.reference_available(), reason="/root/reference not present (GPU box)")
 HERE = os.path.dirname(os.path.abspath(__file__))
+GOLDEN = os.path.join(HERE, "golden", "dropin_engine.npz")
+WEIGHT_SEED = 123
 DISC = {"target": "sgm.modules.diffusionmodules.discretizer.LegacyDDPMDiscretization"}
 # full SDXL widths (LightGLVUNet's 'XL-base' adapter tables are hard-coded for 320 / 640 / 1280 channels, SUPIR_v0.py:560-598) with
 # depth-1 transformers, and both text towers at their real widths with two blocks each: 980 M + 145 M parameters per engine
@@ -105,52 +108,29 @@ def rel_fro(a, b):
 
 @pytest.fixture()
 def backend_on_standins(monkeypatch):
-    """compat.install(conditioner=True) + CPU stand-in kernels + the three `needs CUDA` guards lifted; everything is put back."""
-    import importlib
-    ref_stubs.import_reference()
+    """CPU stand-in kernels + the three `needs CUDA` guards lifted; monkeypatch puts everything back."""
     sys.path.insert(0, HERE)
     import cpu_ops
-    import supir_b200.compat as compat
     from supir_b200 import ops, vae, wrappers
-    saved = {}
-    for modname, attrs in dict(compat.PATCHES, **compat.CONDITIONER_PATCHES).items():
-        m = importlib.import_module(modname)
-        saved.update({(m, a): getattr(m, a) for a in attrs if hasattr(m, a)})
+    cpu_ops.install(monkeypatch)
+    monkeypatch.setattr(vae._VAENet, "_check", lambda self, x: (None if getattr(self, "_packed", False) else self.pack()))
 
-    def activate():
-        cpu_ops.install(monkeypatch)
-        monkeypatch.setattr(vae._VAENet, "_check", lambda self, x: (None if getattr(self, "_packed", False) else self.pack()))
+    def conv1x1(self, x, in_scale=1.0):
+        x = x.float().contiguous()
+        out = torch.empty((x.shape[0], self.out_channels) + tuple(x.shape[2:]), dtype=torch.float32)
+        w = self.weight.detach().reshape(self.out_channels, self.in_channels).to(torch.bfloat16).float().contiguous()
+        return ops.conv1x1_small_nchw(x, w, vae._bias_bf16_values(self.bias), out, in_scale=in_scale)
+    monkeypatch.setattr(vae._Conv1x1Small, "forward", conv1x1)
 
-        def conv1x1(self, x, in_scale=1.0):
-            x = x.float().contiguous()
-            out = torch.empty((x.shape[0], self.out_channels) + tuple(x.shape[2:]), dtype=torch.float32)
-            w = self.weight.detach().reshape(self.out_channels, self.in_channels).to(torch.bfloat16).float().contiguous()
-            return ops.conv1x1_small_nchw(x, w, vae._bias_bf16_values(self.bias), out, in_scale=in_scale)
-        monkeypatch.setattr(vae._Conv1x1Small, "forward", conv1x1)
-
-        def wrapper_forward(self, x, t, c, control_scale=1, context_token=None, **kw):      # ControlWrapper.forward minus the CUDA graph
-            if not self._packed:
-                self.pack()
-            ctx, y = c["crossattn"], c["vector"]
-            plan = wrappers._Plan(self, x.shape[0], x.shape[2], x.shape[3], ctx.shape[1], ctx.shape[2], y.shape[1], "cpu")
-            wrappers.ControlWrapper._fill(plan, x, t, ctx, y, c["control"], control_scale, context_token)
-            plan._run()
-            return plan.out.clone()
-        monkeypatch.setattr(wrappers.ControlWrapper, "forward", wrapper_forward)
-        return compat.install(strict=True, conditioner=True)
-    yield activate
-    for (m, a), v in saved.items():
-        setattr(m, a, v)
-
-
-def build_reference_engine(RS, cfg, tok_l, tok_g):
-    """Pure reference: its conditioner constructors need vocabularies / weights from the network, so the engine is built with the
-    empty conditioner and the real one (tests/golden/make_golden.py:build_reference_conditioner) is attached afterwards."""
-    import make_golden as mg
-    from sgm.modules.encoders import modules as E
-    eng = RS.SUPIRModel(**cfg)
-    eng.conditioner = mg.build_reference_conditioner(E, tok_l, tok_g, ARCH_L, ARCH_G, layer_idx=1)
-    return eng.eval()
+    def wrapper_forward(self, x, t, c, control_scale=1, context_token=None, **kw):      # ControlWrapper.forward minus the CUDA graph
+        if not self._packed:
+            self.pack()
+        ctx, y = c["crossattn"], c["vector"]
+        plan = wrappers._Plan(self, x.shape[0], x.shape[2], x.shape[3], ctx.shape[1], ctx.shape[2], y.shape[1], "cpu")
+        wrappers.ControlWrapper._fill(plan, x, t, ctx, y, c["control"], control_scale, context_token)
+        plan._run()
+        return plan.out.clone()
+    monkeypatch.setattr(wrappers.ControlWrapper, "forward", wrapper_forward)
 
 
 SAMPLING = "sgm.modules.diffusionmodules.sampling."
@@ -184,53 +164,35 @@ def run_scenarios(eng, monkeypatch, untile_reference_hooks=False):
     return out
 
 
-def test_reference_engine_runs_unchanged_on_the_backend(backend_on_standins, monkeypatch):
+def prompt_tokens():
+    """Token ids of every prompt the scenarios use (both towers), in place of the BPE tokenisers."""
+    texts = ["a photo of a cat" + P_P] + [t + P_P for t in LOCAL] + [N_P]
+    return {t: prompt_row(t, 49407) for t in texts}, {t: prompt_row(t, 0) for t in texts}
+
+
+def test_engine_matches_the_reference_engine(backend_on_standins, monkeypatch):
     import contextlib
     import io
     import warnings
-    ref_stubs.import_reference()
-    from SUPIR.models import SUPIR_model as RS
-    texts = ["a photo of a cat" + P_P] + [t + P_P for t in LOCAL] + [N_P]
-    tok_l = {t: prompt_row(t, 49407) for t in texts}
-    tok_g = {t: prompt_row(t, 0) for t in texts}
-    quiet = lambda: contextlib.redirect_stdout(io.StringIO())  # noqa: E731
-    cfg0 = SAMPLING + "RestoreEDMSampler"
-
-    # ---- 1. the reference, untouched ----
-    import SUPIR.modules.SUPIR_v0 as V
-    assert V.GLVControl.__module__ == "SUPIR.modules.SUPIR_v0"
-    with quiet(), warnings.catch_warnings():
+    from supir_b200.model import SUPIRModel
+    ref = np.load(GOLDEN)
+    shapes = json.loads(str(ref["shapes"]))
+    tok_l, tok_g = prompt_tokens()
+    with contextlib.redirect_stdout(io.StringIO()), warnings.catch_warnings():
         warnings.simplefilter("ignore")
-        orig_tensor = torch.tensor
-
-        def cpu_tensor(*a, **k):                                # gaussian_weights hard-codes device='cuda' (sampling.py:750)
-            k.pop("device", None)
-            return orig_tensor(*a, **k)
-        monkeypatch.setattr(torch, "tensor", cpu_tensor)
-        ref = build_reference_engine(RS, engine_config(cfg0, False), tok_l, tok_g)
-        shapes = {k: list(v.shape) for k, v in ref.state_dict().items()}
-        sd = make_state_dict(shapes, seed=123)
-        sd["denoiser.sigmas"] = ref.denoiser.sigmas.clone()     # a persistent buffer, not a weight: keep the real sigma table
-        ref.load_state_dict(sd)
-        want = run_scenarios(ref, monkeypatch, untile_reference_hooks=True)
-        assert type(ref.sampler).__module__ == "sgm.modules.diffusionmodules.sampling"
-    del ref
-
-    # ---- 2. the same class, same config + conditioner config, after compat.install(conditioner=True) ----
-    done = backend_on_standins()
-    assert ("SUPIR.modules.SUPIR_v0", "LightGLVUNet") in done and ("sgm.modules", "GeneralConditionerWithControl") in done
-    with quiet(), warnings.catch_warnings():
-        warnings.simplefilter("ignore")
-        eng = RS.SUPIRModel(**engine_config(cfg0, True)).eval()
+        eng = SUPIRModel(**engine_config(SAMPLING + "RestoreEDMSampler", True)).eval()
         assert type(eng.model).__module__ == "supir_b200.wrappers" and type(eng.conditioner).__module__ == "supir_b200.conditioner"
         assert type(eng.first_stage_model).__module__ == "supir_b200.vae" and type(eng.denoiser).__module__ == "supir_b200.denoiser"
         assert {k: list(v.shape) for k, v in eng.state_dict().items()} == shapes, "state_dict layout differs from the reference engine's"
+        sd = make_state_dict(shapes, seed=WEIGHT_SEED)
+        sd["denoiser.sigmas"] = torch.from_numpy(ref["sigmas"])  # a persistent buffer, not a weight: keep the real sigma table
         eng.load_state_dict(sd)
         eng.conditioner.embedders[0].tokenize = lambda ts: torch.stack([tok_l[t] for t in ts])
         eng.conditioner.embedders[1].tokenize = lambda ts: torch.stack([tok_g[t] for t in ts])
         got = run_scenarios(eng, monkeypatch)
         assert type(eng.sampler).__module__ == "supir_b200.sampling" and type(eng.first_stage_model.decoder.forward).__module__ == "supir_b200.vae"
-    errs = {k: rel_fro(got[k], want[k]) for k in want}
-    print("reference SUPIRModel on the backend, rel. Frobenius vs the pure reference:", {k: f"{v:.4g}" for k, v in errs.items()})
+    assert sorted(got) == sorted(k for k in ref.files if k + "_shape" in ref.files)
+    errs = {k: rel_fro(reference_cases.sample(got[k]), torch.from_numpy(ref[k])) for k in got}
+    print("SUPIRModel on the backend, rel. Frobenius vs the reference engine (seeded sample):", {k: f"{v:.4g}" for k, v in errs.items()})
     for k, v in errs.items():
-        assert got[k].shape == want[k].shape and v <= (3e-2 if k == "stage1_denoise" else 5e-2), (k, v)
+        assert list(got[k].shape) == ref[k + "_shape"].tolist() and v <= (3e-2 if k == "stage1_denoise" else 5e-2), (k, v)

@@ -1,29 +1,22 @@
 """Property tests (hypothesis) of the integer bookkeeping on the hot path — window lists, VAE tile boxes, crops, the window
 partition over ranks, the network-batch grouping. Bit-exact by nature. The product functions are compared with the oracle's
-independent restatement everywhere, and with the LIVE reference functions when /root/reference is present (build container)."""
-import contextlib
-import io
+independent restatement everywhere, and with the reference functions' recorded results on seeded random sizes
+(tests/golden/reference_io.npz, tests/golden/make_reference_io.py)."""
+import json
 import os
 import sys
 
-import pytest
+import numpy as np
 import torch
 from hypothesis import given, settings, strategies as st
 
 sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
-import ref_stubs  # noqa: E402
+import reference_cases  # noqa: E402
 
 from oracle import sampler as osamp, vae as ovae  # noqa: E402
 from supir_b200 import sampling, vae  # noqa: E402
 
-_ref = None
-
-
-def reference():
-    global _ref
-    if _ref is None and ref_stubs.reference_available():
-        _ref = ref_stubs.import_reference()
-    return _ref
+REF = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_io.npz"))
 
 
 @settings(max_examples=200, deadline=None)
@@ -32,9 +25,6 @@ def test_sliding_windows_cover_and_match(tile, stride, dh, dw):
     h, w = tile + dh, tile + dw
     got = sampling._sliding_windows(h, w, tile, stride)
     assert [tuple(c) for c in osamp.sliding_windows(h, w, tile, stride)] == got
-    ref = reference()
-    if ref is not None:
-        assert [tuple(c) for c in ref.sampling._sliding_windows(h, w, tile, stride)] == got
     # every window is a full tile inside the image, rows/cols are covered, order is row-major
     assert all(he - hi == tile and we - wi == tile and 0 <= hi and he <= h and 0 <= wi and we <= w for hi, he, wi, we in got)
     assert got == sorted(got, key=lambda c: (c[0], c[2]))
@@ -51,12 +41,6 @@ def test_split_tiles_and_crops_match(h, w, tile, dec):
     tin, tout = vae.split_tiles(h, w, tile, dec)
     oin, oout = ovae.split_tiles(h, w, tile, dec)
     assert tin == oin and tout == oout
-    ref = reference()
-    if ref is not None:
-        hook = ref.tilevae.VAEHook(None, tile, is_decoder=dec, fast_decoder=False, fast_encoder=False, color_fix=False)
-        with contextlib.redirect_stdout(io.StringIO()):
-            rin, rout = hook.split_tiles(h, w)
-        assert [list(b) for b in rin] == tin and [list(b) for b in rout] == tout
     # output boxes tile the output canvas exactly once (the paste in tiled_forward relies on it)
     H, W = (h * 8, w * 8) if dec else (h // 8, w // 8)
     area = 0
@@ -68,15 +52,39 @@ def test_split_tiles_and_crops_match(h, w, tile, dec):
         th, tw = (th * 8, tw * 8) if dec else (th // 8, tw // 8)
         y0c, y1c, x0c, x1c = vae.crop_margins(th, tw, i, o, dec)
         assert (y0c, y1c, x0c, x1c) == tuple(ovae.crop_margins(th, tw, i, o, dec))
-        if ref is not None and th > 0 and tw > 0 and h >= 8 and w >= 8:
-            idx = torch.arange(th * tw).view(1, 1, th, tw)
-            c = ref.tilevae.crop_valid_region(idx, i, o, dec)
-            assert tuple(c.shape[2:]) == (y1c - y0c, x1c - x0c)
-            if c.numel():
-                assert int(c[0, 0, 0, 0]) == y0c * tw + x0c
     if not dec and (h % 8 or w % 8):
         return              # the reference floors the latent size; exact tiling is only defined for multiples of 8
     assert area == H * W
+
+
+def test_sliding_windows_match_the_reference():
+    """200 seeded random (h, w, tile, stride) over the ranges above: the window list == the reference's _sliding_windows."""
+    want = json.loads(str(REF["sliding_windows"]))
+    cases = reference_cases.sliding_window_cases()
+    assert len(cases) == len(want)
+    for args, (d,) in zip(cases, want):
+        assert reference_cases.digest_list(sampling._sliding_windows(*args)) == d, args
+
+
+def test_split_tiles_and_crops_match_the_reference():
+    """150 seeded random (h, w, tile, decoder) over the ranges above: tile boxes == the reference's VAEHook.split_tiles, and the
+    crop of every tile (size and first element) == the reference's crop_valid_region on an index image."""
+    want = json.loads(str(REF["split_tiles"]))
+    cases = reference_cases.split_tile_cases()
+    assert len(cases) == len(want)
+    for (h, w, tile, dec), (d_in, d_out, d_crop) in zip(cases, want):
+        tin, tout = vae.split_tiles(h, w, tile, dec)
+        assert reference_cases.digest_list(tin) == d_in and reference_cases.digest_list(tout) == d_out, (h, w, tile, dec)
+        crops = []
+        for i, o in zip(tin, tout):
+            th, tw = i[3] - i[2], i[1] - i[0]
+            th, tw = (th * 8, tw * 8) if dec else (th // 8, tw // 8)
+            if th > 0 and tw > 0 and h >= 8 and w >= 8:
+                y0c, y1c, x0c, x1c = vae.crop_margins(th, tw, i, o, dec)
+                crops.append([y1c - y0c, x1c - x0c, y0c * tw + x0c if (y1c - y0c) * (x1c - x0c) > 0 else -1])
+            else:
+                crops.append(None)
+        assert reference_cases.digest_list(crops) == d_crop, (h, w, tile, dec)
 
 
 @settings(max_examples=300, deadline=None)

@@ -12,7 +12,6 @@ import yaml
 from weights import make_state_dict
 
 sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
-import ref_stubs  # noqa: E402
 
 DISC = {"target": "sgm.modules.diffusionmodules.discretizer.LegacyDDPMDiscretization"}
 # construction + checkpoint loading only (no forward pass): a narrow network keeps the files small
@@ -85,16 +84,16 @@ def get_keys(ckpt):
     return ckpt.get("state_dict", ckpt).keys()
 
 
-@pytest.mark.skipif(not ref_stubs.reference_available(), reason="/root/reference not present (GPU box)")
 def test_numpy_helpers_match_the_reference_functions():
+    """HWC3 / Numpy2Tensor against the reference's own functions (SUPIR/util.py), through their recorded outputs
+    (tests/golden/reference_io.npz)."""
+    import reference_cases
     from supir_b200 import util
-    src = open(os.path.join(ref_stubs.REFERENCE_ROOT, "SUPIR", "util.py")).read()
-    ns = {"np": np, "torch": torch}
-    exec(src[src.index("def HWC3"):src.index("def upscale_image")], ns)
-    exec(src[src.index("def Numpy2Tensor"):src.index("def Tensor2Numpy")], ns)
-    rng = np.random.RandomState(0)
-    for shape in ((17, 23), (17, 23, 1), (17, 23, 3), (17, 23, 4)):
-        img = rng.randint(0, 256, shape).astype(np.uint8)
-        assert np.array_equal(util.HWC3(img), ns["HWC3"](img))
-    img = rng.randint(0, 256, (9, 11, 3)).astype(np.uint8)
-    assert torch.equal(util.Numpy2Tensor(img), ns["Numpy2Tensor"](img))
+    ref = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_io.npz"))
+    imgs, img = reference_cases.numpy_helper_inputs()
+    for i, x in enumerate(imgs):
+        want = ref[f"hwc3_{i}"]
+        got = util.HWC3(x)
+        assert got.dtype == want.dtype and np.array_equal(got, want)
+    got = util.Numpy2Tensor(img)
+    assert got.numpy().dtype == ref["numpy2tensor"].dtype and np.array_equal(got.numpy(), ref["numpy2tensor"])
